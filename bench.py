@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark (contract in the task statement; layout in DESIGN.md section 5).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-extras] [--step-path module|functional]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = Correlation forward + backward (both input gradients) at BASELINE.json configs[1]:
@@ -24,6 +25,8 @@ flownet2     : image-pairs/s of the unmodified reference models (random weights,
                of the output flow against the same network on the reference's own kernels, same seeded input,
                deterministic cuDNN, TF32 off (the reference output is computed in a child process: --flow-ref).
 Host staging buffers are allocated after binding the rank to its GPU's NUMA node (flownet2_b200.numa).
+--dump-outputs DIR: rank 0 writes what the last timed step returned (output, grad_input1, grad_input2) as DIR/<name>.npy,
+               float32; the inputs are seeded, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -135,6 +138,23 @@ class ClockSampler:
         self._stop = True
         if self.proc:
             self.proc.terminate()
+
+
+DUMP_ELEMENTS = 1 << 22     # per array: 16 MB of float32, 48 MB for the three outputs of a step
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy in float32: whole if it has at most DUMP_ELEMENTS elements, else the
+    elements at DUMP_ELEMENTS sorted flat indices drawn from a fixed seed (the same positions in every run)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_ELEMENTS:
+            idx = torch.randint(t.numel(), (DUMP_ELEMENTS,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def time_loop(fn, steps, warmup, sync, dist_barrier=None):
@@ -532,6 +552,8 @@ def main():
     ap.add_argument("--flow-ref", nargs="+", metavar=("OUT_DIR", "MODEL"), help=argparse.SUPPRESS)
     ap.add_argument("--step-path", default="module", choices=["module", "functional"],
                     help="ours arm: time the nn.Module + autograd step (default, the call a user makes) or the functional C-ABI calls")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32; a fixed sample of large arrays)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.flow_ref:                      # child of the ours arm: reference-kernel output flows for the agreement check
@@ -593,12 +615,16 @@ def main():
         corr = flownet2_b200.Correlation(CFG["pad"], CFG["k"], CFG["md"], CFG["s1"], CFG["s2"], 1)
         f1.requires_grad_(True)
         f2.requires_grad_(True)
+        last = {}
 
         def step():
             o = corr(f1, f2)
-            torch.autograd.grad(o, (f1, f2), gO)
+            last["output"] = o.detach()
+            last["grad_input1"], last["grad_input2"] = torch.autograd.grad(o, (f1, f2), gO)
         step_how = "flownet2_b200.Correlation module forward + autograd backward (torch.autograd.grad), both input gradients"
     else:
+        last = {"output": out, "grad_input1": g1, "grad_input2": g2}
+
         def step():
             fwd(f1, f2, out)
             bwd(f1, f2, gO, g1, g2)
@@ -609,15 +635,14 @@ def main():
     if rank == 0:
         sampler.start()
     K, Wm = args.steps, args.warmup
-    steps_cap = None
-    if args.impl == "reference":
-        steps_cap = 5            # the reference backward takes ~0.4 s per step: keep the arm within minutes
-        K = min(K, steps_cap)
     l0 = launches()
     step()
     launches_timed = (launches() - l0) * K      # kernels launched per step x timed steps
     ms, t0, t1 = time_loop(step, K, Wm, sync, barrier if dist else None)
     clocks = sampler.window(t0, t1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:         # before the kernel timings below overwrite out / g1 / g2
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
 
     # dominant-kernel timing (alone, same stream): forward kernel, backward kernels
     f1, f2 = f1.detach(), f2.detach()
@@ -642,7 +667,6 @@ def main():
 
     def e2e_step():
         pipe.submit(e2e_compute, (hf1, hf2, hgO), (hout, hg1, hg2))
-    Ke = min(K, 40)
     for _ in range(2):
         e2e_step()
     pipe.drain()
@@ -651,7 +675,7 @@ def main():
     sync()
     ee0, ee1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ee0.record()
-    for _ in range(Ke):
+    for _ in range(K):
         e2e_step()
     pipe.drain()
     ee1.record()
@@ -661,12 +685,12 @@ def main():
     ms_e = ee0.elapsed_time(ee1)
     e2e_check = float((hg1 - g1.cpu()).abs().max()) if args.impl == "ours" else 0.0   # same inputs -> same result as the resident step
 
-    stats = torch.tensor([ms, ms_e / Ke * K], device=dev, dtype=torch.float64)
+    stats = torch.tensor([ms, ms_e], device=dev, dtype=torch.float64)
     stats_min = stats.clone()
     if dist:
         dist.all_reduce(stats, op=dist.ReduceOp.MAX)
         dist.all_reduce(stats_min, op=dist.ReduceOp.MIN)
-    ms, ms_e_scaled = float(stats[0]), float(stats[1])
+    ms, ms_e = float(stats[0]), float(stats[1])
     ms_fastest_rank = float(stats_min[0])
 
     # second half of BASELINE.json's metric: FlowNet2 image-pairs/sec (every rank runs a replica)
@@ -706,7 +730,7 @@ def main():
     fwd_b, bwd_b, bwd_launch_b = alg_bytes(B)
     total_b = (fwd_b + bwd_b) * world
     value = total_b * K / (ms * 1e-3) / 1e9
-    e2e_value = total_b * K / (ms_e_scaled * 1e-3) / 1e9
+    e2e_value = total_b * K / (ms_e * 1e-3) / 1e9
     peak, peak_src = measured_peak()
 
     if rank == 0:
@@ -755,7 +779,7 @@ def main():
             "kernels": {"forward_ms": round(per_f, 4), "backward_ms": round(per_b, 4),
                         "forward_GBps": round(fwd_b / per_f / 1e6, 1), "backward_GBps": round(bwd_b / per_b / 1e6, 1)},
             "e2e": {"value": round(e2e_value, 2), "unit": "GB/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                    "ms_per_step": round(ms_e_scaled / K, 3), "steps": Ke,
+                    "ms_per_step": round(ms_e / K, 3), "steps": K,
                     "how": "flownet2_b200.hostpipe.HostPipeline: pinned host buffers, H2D / kernels / D2H of consecutive "
                            "steps on three streams, 2 device buffer sets", "max_abs_diff_vs_resident": e2e_check},
             "gpu_launches": int(launches_timed),
@@ -766,7 +790,6 @@ def main():
         if args.impl == "reference":
             line["impl"] = "reference"
             line["config"]["impl"] = "reference CUDA kernels rebuilt for sm_100a (oracle/_ref)"
-            line["steps_requested"], line["steps_cap"] = args.steps, steps_cap
         if world == 1:
             try:
                 line["cpu_baseline"] = cpu_baseline_sample()
